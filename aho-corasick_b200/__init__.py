@@ -422,12 +422,15 @@ class AhoCorasick:
     def __init__(self, handle):
         self._h = handle
         self._cap_hint = 4096  # output-buffer sizing for the two-call overflow protocol
+        # freed by the library that made it: the CPU dry-run library of tests/emu/ can stand in for
+        # `_lib` while handles made by the other one are still alive
+        self._free = _lib.acg_dfa_free
 
     def __del__(self):
         h = getattr(self, "_h", None)
         if h and _lib is not None:
             try:
-                _lib.acg_dfa_free(h)
+                self._free(h)
             except Exception:
                 pass
             self._h = None

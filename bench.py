@@ -3,7 +3,12 @@
 MatchKind::Standard overlapping) on N B200s, with roofline / cpu_baseline / e2e objects.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--hay-gib G] [--workload cfg2|cfg3|cfg4|cfg5]
-                    [--impl reference]
+                    [--impl reference] [--dump-outputs DIR]
+
+Every timed loop (the workload's device-resident steps, its end-to-end steps and those of the extra
+configs) runs exactly K steps.  --dump-outputs DIR writes the matches the last timed step of the
+workload returned to its caller (see dump_outputs) so that two builds can be compared on the same
+seeded inputs.
 
 Our arm: every search goes through the C ABI of libacb200.so (ctypes).  N > 1: one process per GPU,
 acg_comm_init + acg_find_overlapping_sharded (haystack slices, records stored into rank 0's buffer
@@ -136,6 +141,31 @@ def bind_to_gpu_numa_node(local_rank):
     return None
 
 
+DUMP_BYTES = 64_000_000 - 4096   # 64 MB in all, npy headers included
+DUMP_SEED = 0xD0AC
+
+
+def dump_outputs(out_dir, rec):
+    """The match records (pid, start, end in global offsets, in the order the caller receives them)
+    as float64 arrays -- exact, offsets stay far below 2^53 -- in out_dir/{pid,start,end}.npy, with
+    out_dir/match_count.npy.  A list too large for DUMP_BYTES is cut to a fixed seeded sample of
+    records, in order; out_dir/sample_index.npy then holds their positions in the full list."""
+    import numpy as np
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    n = len(rec)
+    arrays = {"match_count": np.array([n], dtype=np.float64)}
+    if n * 3 * 8 > DUMP_BYTES:
+        keep = DUMP_BYTES // (4 * 8)
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(n, size=keep, replace=False))
+        rec = rec[idx]
+        arrays["sample_index"] = idx.astype(np.float64)
+    for k in ("pid", "start", "end"):
+        arrays[k] = rec[k].astype(np.float64)
+    for name, a in arrays.items():
+        np.save(out_dir / f"{name}.npy", a)
+
+
 def cpu_scan(o, hay, cores, back):
     """One pass of the oracle's overlapping DFA loop over `hay` on `cores` threads (slices with
     max_pattern_len-1 overlap; the C call releases the GIL).  Returns the match count."""
@@ -247,8 +277,9 @@ class Rig:
         return int(t.item())
 
 
-def run_workload(rig, args, wl, steps, warmup, want_e2e=True, check=True):
-    """Device-resident and end-to-end throughput of one workload on rig.world GPUs."""
+def run_workload(rig, args, wl, steps, warmup, want_e2e=True, check=True, dump_dir=None):
+    """Device-resident and end-to-end throughput of one workload on rig.world GPUs; with dump_dir,
+    rank 0 writes what the last timed step returned there (dump_outputs)."""
     import numpy as np
     import aho_corasick_b200 as ab
     from aho_corasick_b200 import sharded as S
@@ -304,6 +335,7 @@ def run_workload(rig, args, wl, steps, warmup, want_e2e=True, check=True):
                 else:
                     r, ms = ac.find_iter_dev_np(d_hay.data_ptr(), n_local, span)
                     n = len(r)
+                    state["found"] = r
                 return n, ms, 0.0, None
             except OverflowError as e:
                 state["cap"] = int(e.args[0]) * 9 // 8 + 1024
@@ -370,6 +402,17 @@ def run_workload(rig, args, wl, steps, warmup, want_e2e=True, check=True):
                 gather_ms.append(gms)
         rig.barrier()
         wall = time.perf_counter() - t0
+    if dump_dir is not None and rank == 0:
+        # N > 1: every rank's records in rank 0's buffer; N = 1: the ordered records left on the device
+        # (overlapping) or the list returned (find_iter)
+        if world > 1:
+            last = rig.comm.fetch()
+        elif overlapping:
+            last = state["out"][: cnt * ab.MATCH_DTYPE.itemsize].cpu().numpy().view(ab.MATCH_DTYPE)
+        else:
+            last = state["found"]
+        dump_outputs(dump_dir, last)
+        del last
     stats = ac.last_stats()
     if mode == "stream":
         # one pair of CUDA events around the K overlapped steps, taken inside the library after the
@@ -420,12 +463,11 @@ def run_workload(rig, args, wl, steps, warmup, want_e2e=True, check=True):
         for _ in range(2):
             n_e2e = e2e_step(h_np)
         rig.barrier()
-        e2e_steps = max(2, min(steps, 4))
         t0 = time.perf_counter()
-        for _ in range(e2e_steps):
+        for _ in range(steps):
             n_e2e = e2e_step(h_np)
         rig.barrier()
-        (e2e_s,) = rig.max_over_ranks((time.perf_counter() - t0) / e2e_steps)
+        (e2e_s,) = rig.max_over_ranks((time.perf_counter() - t0) / steps)
         e2e = {"value": world * e2e_bytes / GIB / e2e_s, "unit": "GiB/s", "h2d_bytes_per_step": e2e_bytes,
                "d2h_bytes_per_step": int(n_e2e * 24), "host_memory": "pinned",
                "call": "acg_find_overlapping_sharded(host slice)" if world > 1 else
@@ -437,8 +479,9 @@ def run_workload(rig, args, wl, steps, warmup, want_e2e=True, check=True):
             p_np[:] = h_np
             e2e_step(p_np)
             t0 = time.perf_counter()
-            e2e_step(p_np)
-            e2e["pageable_value"] = e2e_bytes / GIB / (time.perf_counter() - t0)
+            for _ in range(steps):
+                e2e_step(p_np)
+            e2e["pageable_value"] = e2e_bytes / GIB / ((time.perf_counter() - t0) / steps)
             del p_np
         del h_hay, h_np
     scan_s = sum(scan_ms) / len(scan_ms) / 1e3
@@ -507,7 +550,13 @@ def main():
     ap.add_argument("--host-fill", action="store_true", help="cfg5: build the dense table on the host")
     ap.add_argument("--experiment", type=int, default=0,
                     help="ACG_EXP_* flags (include/acb200_debug.h); 0 = default kernel")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the matches of the workload's last timed step to DIR/*.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.warmup < 0:
+        ap.error("--warmup must not be negative")
     if args.impl == "reference":
         return reference_arm(args)
 
@@ -515,7 +564,7 @@ def main():
     rig = Rig(args)
     world, rank = rig.world, rig.rank
     wl = args.workload
-    main_res = run_workload(rig, args, wl, args.steps, args.warmup, want_e2e=True)
+    main_res = run_workload(rig, args, wl, args.steps, args.warmup, want_e2e=True, dump_dir=args.dump_outputs)
     extras = {}
     if not args.no_extras and not args.experiment and wl == "cfg2":
         # the other BASELINE configs, device-resident, so that the driver-run line carries them:
@@ -523,7 +572,7 @@ def main():
         for x in (["cfg3", "cfg4", "cfg5"] if world == 1 else ["cfg5"]):
             saved = args.no_cpu_baseline
             args.no_cpu_baseline = True
-            r = run_workload(rig, args, x, max(3, min(args.steps, 5)), 3, want_e2e=(x == "cfg5" and world > 1), check=True)
+            r = run_workload(rig, args, x, args.steps, 3, want_e2e=(x == "cfg5" and world > 1), check=True)
             args.no_cpu_baseline = saved
             extras[x] = r
     if rank != 0:
