@@ -9,6 +9,7 @@ import aho_corasick_b200 as ab
 import golden_util as G
 import oracle_py as O
 from aho_corasick_b200 import workload as W
+from test_prefilter_plan import set_experiment
 
 pytestmark = pytest.mark.gpu
 
@@ -310,6 +311,12 @@ def test_full_size_properties_config2():
     assert (cnt_p, fnv_p) == (cnt_w, fnv_w)
     assert cnt_p >= planted
     ac.set_engine(ab.Engine.Auto)
+    # global super-tiles (ACG_EXP_GLOBAL_TILES = 16): one chunk spans the whole 4 GiB region, so the
+    # kernel's queued 32-bit offsets go through its 2 GiB windows
+    set_experiment(ac, 16)
+    assert ac.count_overlapping_dev(d.data_ptr(), n)[:2] == (cnt_p, fnv_p)
+    assert ac.last_stats()["engine"] == int(ab.Engine.Prefilter)
+    set_experiment(ac, 0)
     full, _ = ac.find_overlapping_iter_dev_np(d.data_ptr(), n)
     assert len(full) == cnt_p
     cut = (2 << 30) + 12345
